@@ -1,8 +1,12 @@
 #!/usr/bin/env python
 """bench.py -- headline metric of BASELINE.json: SGEMM TFLOP/s (2*M*N*K / t) at M=N=K=8192.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   (N > 1: launched by torch.distributed.run, one rank per GPU)
+
+--dump-outputs DIR writes the C of the last timed step (the array the caller of the headline path receives) as
+DIR/C.npy (DIR/C_rank<r>.npy per rank at N > 1), float32: the same seeded sample of DUMP_ROWS rows in every run, 32 MB
+in all.  The inputs are seeded, so two builds given the same arguments can be compared output for output.
 
 A "step" is one pass of the hot path: C <- A x B, fp32, row-major, alpha=1, beta=0 (the call the reference's bench
 makes, benchmarks/gemm/gemm_bench_float32.nim:184-189), through the C ABI of liblaser_b200.so in its DEFAULT fp32 mode
@@ -35,6 +39,13 @@ METRIC = "sgemm_tflops_m8192_n8192_k8192"
 UNIT = "TFLOP/s"
 MNK = 8192
 STRONG_M = 32768
+DUMP_ROWS = 1024      # rows of C written by --dump-outputs, over all ranks: 1024 x 8192 fp32 = 32 MB
+
+
+def dump_rows(M, world):
+    """indices of the rows of one rank's C that --dump-outputs writes: the same seeded sample in every run"""
+    import numpy as np
+    return np.sort(np.random.default_rng(0).choice(M, DUMP_ROWS // world, replace=False))
 
 
 def load_traffic():
@@ -344,6 +355,10 @@ def run_ours(args):
     n0 = L.launch_count()
     ms_step = timed(step, args.steps, 0)
     launches = L.launch_count() - n0
+    dump = None
+    if args.dump_outputs:
+        # read before the profiled and untimed steps below run the product again
+        dump = C.view(M, N)[torch.as_tensor(dump_rows(M, world), device=dev)].cpu().numpy()
     # kernel-level roofline numbers: the same step, bracketed by CUDA events inside the library (profile mode disables the
     # dependent launch of the GEMM kernel, so it is measured separately from the headline time above)
     L.profile_begin()
@@ -469,6 +484,10 @@ def run_ours(args):
            "h2d_bytes_per_step": (M * K + K * N) * 4 * world, "d2h_bytes_per_step": M * N * 4 * world,
            "api": "laser_b200_gemm_strided_f32 (host pointers, reference signature), pinned host buffers, steps=%d" % e2e_steps}
 
+    if dump is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "C.npy" if world == 1 else "C_rank%d.npy" % rank), dump)
+
     ok = parity["ok"] and (strong_parity is None or strong_parity["ok"])
     if rank == 0:
         cpu = cpu_reference_sample() if world == 1 else None
@@ -546,7 +565,12 @@ def main():
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the C of the last timed step (a seeded sample of rows) as .npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)
