@@ -47,9 +47,23 @@ def test_parity_file_subset_against_the_host_emulated_library():
     """tests/test_gpu_parity.py is backend-neutral (tests/backend.py): the same assertions the B200 has to
     meet -- known-answer vectors on every path and dtype, bit-exactness of the exact kernel, bf16, the
     host-pointer entry, dispatch, the Tensor contract -- are checked here on the CPU build.  A fast
-    subset by default; LASER_B200_EMU_FULL=1 runs the whole parity, fuzz, pre-packed and fused-epilogue
-    files (about 18 minutes: 718 cases passed when last run, 34 skipped for size)."""
+    subset by default; LASER_B200_EMU_FULL=1 runs the whole parity, fuzz, pre-packed, fused-epilogue,
+    epilogue-path and few-rows / GEMV files (about 12 minutes on 8 cores, sizes too large for the CPU build skipped)."""
     assert _run_gpu_files(["test_gpu_parity.py"], ["-k", FAST], 1500) >= 50
+
+
+# fast subsets of the epilogue-path and few-rows / GEMV files: the fused epilogue on the exact and few-rows kernels and on the
+# split-K reduce (100 x 520 x 1024 splits in two under the emulation's default 8 SMs), the few-rows kernels, GEMV below
+# 20000 rows
+EPILOGUE_FAST = "exact_kernel_epilogue or split_single_k1024-col-relu or split_single_k1024-row-tanh or planner"
+FEW_ROWS_FAST = "kernel_selection or random or batched or host_pointer or (gemv and M1031)"
+
+
+def test_epilogue_and_few_rows_files_subset_against_the_host_emulated_library():
+    """tests/test_gpu_epilogue_paths.py and tests/test_gpu_few_rows_gemv.py: a fast subset by default (the whole files with
+    LASER_B200_EMU_FULL=1 below)"""
+    assert _run_gpu_files(["test_gpu_epilogue_paths.py"], ["-k", EPILOGUE_FAST], 1500) >= 60
+    assert _run_gpu_files(["test_gpu_few_rows_gemv.py"], ["-k", FEW_ROWS_FAST], 1500) >= 60
 
 
 def test_f16x3_mode_file_against_the_host_emulated_library():
@@ -57,7 +71,7 @@ def test_f16x3_mode_file_against_the_host_emulated_library():
     assert _run_gpu_files(["test_gpu_zy_f16x3_mode.py"], [], 1500) >= 40
 
 
-@pytest.mark.skipif(os.environ.get("LASER_B200_EMU_FULL", "0") != "1", reason="about 18 minutes; set LASER_B200_EMU_FULL=1")
+@pytest.mark.skipif(os.environ.get("LASER_B200_EMU_FULL", "0") != "1", reason="about 12 minutes; set LASER_B200_EMU_FULL=1")
 def test_whole_parity_and_fuzz_files_against_the_host_emulated_library():
-    assert _run_gpu_files(["test_gpu_parity.py", "test_gpu_fuzz.py", "test_gpu_prepacked.py", "test_gpu_fused_epilogue.py"], [],
-                          5000) >= 700
+    assert _run_gpu_files(["test_gpu_parity.py", "test_gpu_fuzz.py", "test_gpu_prepacked.py", "test_gpu_fused_epilogue.py",
+                           "test_gpu_epilogue_paths.py", "test_gpu_few_rows_gemv.py"], [], 9000) >= 850

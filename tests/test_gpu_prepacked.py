@@ -5,8 +5,8 @@ import numpy as np
 import pytest
 
 import oracle as O
-from backend import dev, sync
-from util import embed, golden_cases
+from backend import dev, emu_budget, sync
+from util import embed, extract, golden_cases
 
 pytestmark = pytest.mark.gpu
 import laser_b200 as L  # noqa: E402
@@ -49,6 +49,31 @@ def test_packed_matches_oracle_and_unpacked(la, lb):
     assert O.max_relative_error(got, want) < 1e-4
     # same tiles, same order of accumulation: packing changes nothing numerically
     assert np.array_equal(got, tC2.cpu().numpy()) and np.array_equal(got, tC3.cpu().numpy())
+
+
+@pytest.mark.parametrize("lc", ["row", "col"])
+@pytest.mark.parametrize("shape", [(100, 520, 777), (300, 520, 4096)], ids=["single_cta", "split_k"])
+def test_packed_single_cta_split_k_and_col_major_c(shape, lc):
+    """a single-CTA tile (M <= 128) and a split-K product (partial planes reduced by a second kernel), C row- or
+    column-major: packed A and B, packed B only and the unpacked F16X3 call agree bit for bit"""
+    M, N, K = shape
+    emu_budget(float(M) * N * K)
+    A = O.fill_uniform_f32(M * K, 94, -1, 1).reshape(M, K); B = O.fill_uniform_f32(K * N, 95, -1, 1).reshape(K, N)
+    C0 = O.fill_uniform_f32(M * N, 96, -1, 1).reshape(M, N)
+    bc, oc, rsc, csc = embed(C0, lc)
+    tA, tB = dev(A), dev(B)
+    pa, pb = pack_both(M, N, K, tA, 0, K, 1, tB, 0, N, 1)
+    outs = [dev(bc) for _ in range(3)]
+    L.gemm_packed(M, N, K, 0.5, pa, pb, -1.25, outs[0], rsc, csc)
+    L.gemm_packedB(M, N, K, 0.5, tA, K, 1, pb, -1.25, outs[1], rsc, csc)
+    L.gemm_strided(M, N, K, 0.5, tA, K, 1, tB, N, 1, -1.25, outs[2], rsc, csc, path=L.PATH_F16X3)
+    sync()
+    got = [extract(t.cpu().numpy(), oc, rsc, csc, M, N) for t in outs]
+    scale = 0.5 * (np.abs(A.astype(np.float64)) @ np.abs(B.astype(np.float64))) + 1.25 * np.abs(C0)
+    ref = 0.5 * (A.astype(np.float64) @ B.astype(np.float64)) - 1.25 * C0
+    assert np.max(np.abs(got[0] - ref) / scale) < 1e-4
+    assert np.array_equal(got[0].view(np.uint32), got[1].view(np.uint32))
+    assert np.array_equal(got[0].view(np.uint32), got[2].view(np.uint32))
 
 
 def test_mem_required_and_reuse():
