@@ -359,6 +359,28 @@ int laser_b200_conv2d_im2col_f32(float *output, const float *input, const int64_
                                  const float *kernel, const int64_t kshape[4], const int64_t padding[2],
                                  const int64_t strides[2]);
 
+/* direct convolution (benchmarks/convolution/conv2d_direct_convolution.nim:8-76): the same shapes as
+ * conv2d_im2col (validated by the same checks), no workspace, ONE kernel launch per call whatever the batch
+ * (none for a batch of 0, which leaves `output` untouched).  Every output element is bit for bit what
+ * laser_b200_conv2d_im2col_f32_dev(..., path = LASER_B200_PATH_SIMT) returns: one FMA chain from +0 over
+ * ascending tap kk = (ci*kH + kr)*kW + kc inside blocks of 512 taps, the blocks added in order.
+ * epi: NULL, or bias = NULL / a device vector of c_out values (requires bias_per_row = 1) and an activation
+ * 0..3, applied once to the final sum as act(x + bias[co]) -- the values im2col followed by
+ * laser_b200_gemm_strided_f32_epi_dev(path SIMT, bias_per_row = 1) gives.  Anything else: EINVAL.
+ * Deliberate departures from the reference:
+ *   - `output` is overwritten and never read (the reference adds into a zero-initialised `oim`);
+ *   - the output column steps the input by the WIDTH stride (the reference multiplies it by the height
+ *     stride, conv2d_direct_convolution.nim:61, which differs for non-square strides);
+ *   - taps outside the image contribute fma(0, w) like the zeros of the im2col workspace (the reference
+ *     skips them), so an infinite weight makes the border outputs NaN exactly as conv2d_im2col does. */
+int laser_b200_conv2d_direct_f32_dev(float *output, const float *input, const int64_t ishape[4],
+                                     const float *kernel, const int64_t kshape[4], const int64_t padding[2],
+                                     const int64_t strides[2], const laser_b200_epilogue *epi, void *stream);
+/* host pointers, synchronous, no epilogue: the reference's conv2d_direct signature */
+int laser_b200_conv2d_direct_f32(float *output, const float *input, const int64_t ishape[4],
+                                 const float *kernel, const int64_t kshape[4], const int64_t padding[2],
+                                 const int64_t strides[2]);
+
 /* dst <- src over a common shape, any strides (device tensor views of the same dtype and shape):
  * copyFrom of laser/tensor/initialization.nim:80-112 (contiguous pairs take a plain device copy,
  * the rest the strided kernel -- the reference's forEachStrided d in dst, s in src: d = s). */

@@ -17,6 +17,7 @@
 //   laser::TensorShape/KernelShape/Padding/Strides, conv2d_out_shape, im2col_workspace_size,
 //   conv2d_im2col                                     benchmarks/convolution/conv2d_common.nim:6-45,
 //                                                     conv2d_im2col.nim:8-166
+//   conv2d_direct                                     conv2d_direct_convolution.nim:8-76
 #pragma once
 
 #include <cstdint>
@@ -244,6 +245,17 @@ inline void conv2d_im2col(float *output, TensorShape oshape, const float *input,
   const int64_t is[4] = {ishape.n, ishape.c, ishape.h, ishape.w}, ks[4] = {kshape.c_out, kshape.c_in, kshape.kH, kshape.kW};
   const int64_t pd[2] = {padding.h, padding.w}, st[2] = {strides.h, strides.w};
   check(laser_b200_conv2d_im2col_f32(output, input, is, kernel, ks, pd, st));
+}
+// conv2d_direct_convolution.nim:8-76 with the same arguments: no workspace, one kernel launch, output fully overwritten
+// (the reference adds into a zeroed output), bit for bit the values of conv2d_im2col on the exact path.
+inline void conv2d_direct(float *output, TensorShape oshape, const float *input, TensorShape ishape, const float *kernel,
+                          KernelShape kshape, Padding padding, Strides strides) {
+  const TensorShape expect = conv2d_out_shape(ishape, kshape, padding, strides);
+  if (expect.n != oshape.n || expect.c != oshape.c || expect.h != oshape.h || expect.w != oshape.w)
+    throw std::invalid_argument("conv2d_direct: oshape does not match conv2d_out_shape");
+  const int64_t is[4] = {ishape.n, ishape.c, ishape.h, ishape.w}, ks[4] = {kshape.c_out, kshape.c_in, kshape.kH, kshape.kW};
+  const int64_t pd[2] = {padding.h, padding.w}, st[2] = {strides.h, strides.w};
+  check(laser_b200_conv2d_direct_f32(output, input, is, kernel, ks, pd, st));
 }
 
 }  // namespace laser

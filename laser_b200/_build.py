@@ -14,7 +14,7 @@ LIB_DIR = os.path.join(_HERE, "lib")
 OBJ_DIR = os.path.join(LIB_DIR, "obj")
 LIB_PATH = os.path.join(LIB_DIR, "liblaser_b200.so")
 SOURCES = ["capi.cu", "tc_f16x3.cu", "tc_tf32x3.cu", "tc_tf32x1.cu", "tc_bf16.cu"]
-HEADERS = ["ptx.cuh", "f16_scale.cuh", "gemm_tc.cuh", "tc_params.h", "tc_launch.h", "tc_launch_impl.cuh", "gemm_simt.cuh", "gemm_dmma.cuh",
+HEADERS = ["ptx.cuh", "f16_scale.cuh", "gemm_tc.cuh", "tc_params.h", "tc_launch.h", "tc_launch_impl.cuh", "gemm_simt.cuh", "simt_epilogue.cuh", "gemm_dmma.cuh",
            "gemm_simt_kernel.inc", "split.cuh", "layers.cuh", "capi_layers.inc", "capi_multi.inc",
            "../../include/laser_b200.h"]
 

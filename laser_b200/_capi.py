@@ -108,6 +108,9 @@ SIGNATURES = {
     "laser_b200_conv2d_im2col_f32_dev": (ctypes.c_int, [vp, vp, i64 * 4, vp, i64 * 4, i64 * 2, i64 * 2, vp, i64,
                                                         ctypes.c_int, vp]),
     "laser_b200_conv2d_im2col_f32": (ctypes.c_int, [vp, vp, i64 * 4, vp, i64 * 4, i64 * 2, i64 * 2]),
+    "laser_b200_conv2d_direct_f32_dev": (ctypes.c_int, [vp, vp, i64 * 4, vp, i64 * 4, i64 * 2, i64 * 2, ctypes.POINTER(Epilogue),
+                                                        vp]),
+    "laser_b200_conv2d_direct_f32": (ctypes.c_int, [vp, vp, i64 * 4, vp, i64 * 4, i64 * 2, i64 * 2]),
     "laser_b200_copy_views": (ctypes.c_int, [ctypes.POINTER(TensorView), ctypes.POINTER(TensorView), vp]),
     "laser_b200_foreach_views": (ctypes.c_int, [ctypes.c_int, ctypes.POINTER(TensorView), ctypes.POINTER(TensorView),
                                                 ctypes.POINTER(TensorView), ctypes.POINTER(TensorView), f64, vp]),

@@ -24,6 +24,7 @@
 #include <type_traits>
 
 #include "ptx.cuh"
+#include "simt_epilogue.cuh"
 
 namespace lb200 {
 
@@ -98,20 +99,6 @@ inline int64_t simt_plan(SimtParams<T> &p, int64_t M, int64_t N, int64_t K, T al
   return mblocks * nblocks;
 }
 
-// bias + activation of the fused epilogue, out of line: inlined into the unrolled MT x NC store loops the tanhf / expf bodies
-// made the kernels several times larger than the instruction cache (ncu: 58 % of the stall samples "no instruction")
-#ifndef LB200_HOST_EMULATION
-static __device__ __noinline__
-#else
-inline
-#endif
-float simt_bias_act(float x, const float *bias, int bias_per_row, int act, int64_t row, int64_t col) {
-  if (bias) x += bias_per_row ? bias[row] : bias[col];
-  if (act == 1) x = fmaxf(x, 0.0f);
-  else if (act == 2) x = tanhf(x);
-  else if (act == 3) x = 1.0f / (1.0f + expf(-x));
-  return x;
-}
 #ifndef LB200_SIMT_MINB
 #define LB200_SIMT_MINB 1
 #endif
@@ -125,15 +112,6 @@ float simt_bias_act(float x, const float *bias, int bias_per_row, int act, int64
 #include "gemm_simt_kernel.inc"
 #undef LB200_SIMT_KERNEL_NAME
 #undef LB200_SIMT_BATCHED
-
-// dynamic shared memory (tests/emu runs this header on host threads, where it is a plain buffer)
-#ifndef LB200_DYN_SMEM
-#ifdef LB200_HOST_EMULATION
-#define LB200_DYN_SMEM(T, name) T *name = reinterpret_cast<T *>(emu::dyn_smem_ptr())
-#else
-#define LB200_DYN_SMEM(T, name) extern __shared__ T name[]
-#endif
-#endif
 
 // ---------------------------------------------------------------------------
 // Skinny GEMM: N <= 4 (matrix x few vectors).  One warp per output row: lanes stride

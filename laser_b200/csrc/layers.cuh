@@ -1,13 +1,16 @@
 // layers.cuh -- the HBM-bound steps either side of the GEMM in the reference's intended use
 // (SURVEY.md section 8f, rank 4): physical transposition / NCHW<->NHWC
-// (laser/primitives/swapaxes.nim:16-112), im2col (benchmarks/convolution/conv2d_im2col.nim:44-93)
-// and the strided N-d copy behind copyFrom (laser/tensor/initialization.nim:80-112).
+// (laser/primitives/swapaxes.nim:16-112), im2col (benchmarks/convolution/conv2d_im2col.nim:44-93),
+// the direct convolution (benchmarks/convolution/conv2d_direct_convolution.nim:8-76) and the strided N-d copy behind
+// copyFrom (laser/tensor/initialization.nim:80-112).
 // All of them move each byte once: coalesced 16-byte global accesses where the shapes allow,
 // shared-memory tiles for the transposition, grids sized from the SM count by the host.
 #pragma once
 
 #include <cuda_runtime.h>
 #include <stdint.h>
+
+#include "simt_epilogue.cuh"
 
 namespace lb200 {
 
@@ -158,6 +161,225 @@ im2col_kernel(float *__restrict__ ws, const float *__restrict__ in, Im2colParams
 #pragma unroll
       for (int e = 0; e < 4; ++e)
         if (p0 + e < p.outHW) dst[e] = v[e];
+    }
+  }
+}
+
+// ---- direct convolution: images x [C][H][W] (*) [Cout][C][kH][kW] -> images x [Cout][outH][outW], no workspace ----
+// Every output is the value the exact im2col path computes (im2col_kernel, then the exact GEMM with M = Cout, K = C*kH*kW,
+// N = outH*outW): one __fmaf_rn chain from +0 over ascending tap kk = (ci*kH + kr)*kW + kc inside blocks of DC_KC taps,
+// the blocks summed in order (x = 0 + blk0, x = x + blk1, ...), taps outside the image multiplied as zeros, and the bias +
+// activation applied once to the final sum through simt_bias_act (bias per output channel = per GEMM row).
+//
+// Work unit ("tile"): DC_PIX consecutive output pixels (flattened oh * outW + ow) of one image x DC_CG output channels; a
+// 1-d grid strides over images x tiles x channel groups (decoded in 64 bits).  Thread t owns the pixels p0 + t + j*256,
+// j < DC_CPT, so every store of a warp writes 32 consecutive floats of one output plane (one 128-byte line) and the
+// staged-input reads of a warp hit consecutive shared-memory words.  It keeps DC_CPT x DC_CG running sums (and as many
+// block totals when K > DC_KC) in registers.
+//   STAGED: per chunk of `cc` input channels the rows the tile's taps touch are copied to shared memory at full padded
+//           width, zero outside the image, next to the chunk's weights of the channel group ([tap][co], two 16-byte
+//           broadcast reads per tap) and a table of each tap's offset inside the staged window.
+//   not STAGED (a single staged channel would exceed DC_SMEM_BYTES: very wide images): weights in 512-tap chunks, input
+//           read from global memory with a bounds check per tap.
+constexpr int DC_CG = 8;                // output channels per group
+constexpr int DC_CPT = 4;               // pixels per thread
+constexpr int DC_PIX = 256 * DC_CPT;    // pixels per tile
+constexpr int DC_KC = 2048 / 4;         // taps per summation block: the exact GEMM's kc (gemm_tiling.nim:310)
+constexpr int DC_SMEM_BYTES = 48 * 1024;   // static shared memory of one block (3 blocks fit an SM's 227 KB)
+
+struct DirectConvParams {
+  int C, H, W, Cout, kH, kW, pH, pW, sH, sW, outH, outW;
+  int K, khw, outHW;
+  int tiles, groups;       // pixel tiles per image, channel groups
+  int64_t total;           // images * tiles * groups
+  int cc;                  // STAGED: input channels per chunk
+  int rows, pitch, plane;  // STAGED: staged rows per channel, row pitch (floats), rows * pitch
+  int ws_off, toff_off;    // STAGED: float offsets of the weights and of the tap-offset table in shared memory
+  const float *bias;       // NULL or Cout values (device)
+  int act;                 // 0 none, 1 relu, 2 tanh, 3 sigmoid
+};
+
+// host side: launch geometry.  geom = {C, H, W, Cout, kH, kW, pH, pW, sH, sW, outH, outW} (checked by conv_geom).
+// Returns whether the STAGED variant of the kernel applies (always false with stage_input = false: the variant that reads
+// the input from global memory, which the library takes only when one staged channel does not fit DC_SMEM_BYTES).
+inline bool direct_conv_plan(const int64_t geom[12], int64_t images, DirectConvParams *p, bool stage_input = true) {
+  p->C = (int)geom[0]; p->H = (int)geom[1]; p->W = (int)geom[2]; p->Cout = (int)geom[3];
+  p->kH = (int)geom[4]; p->kW = (int)geom[5]; p->pH = (int)geom[6]; p->pW = (int)geom[7];
+  p->sH = (int)geom[8]; p->sW = (int)geom[9]; p->outH = (int)geom[10]; p->outW = (int)geom[11];
+  p->khw = p->kH * p->kW;
+  p->K = p->C * p->khw;
+  p->outHW = p->outH * p->outW;
+  p->tiles = (p->outHW + DC_PIX - 1) / DC_PIX;
+  p->groups = (p->Cout + DC_CG - 1) / DC_CG;
+  p->total = images * p->tiles * p->groups;
+  p->bias = nullptr;
+  p->act = 0;
+  // output rows a tile of DC_PIX consecutive pixels can touch, hence input rows and the padded width it needs
+  const int64_t pix = p->outHW < DC_PIX ? p->outHW : DC_PIX;
+  int64_t span = (pix - 1 + p->outW - 1) / p->outW + 1;
+  if (span > p->outH) span = p->outH;
+  const int64_t rows = (span - 1) * geom[8] + geom[4], pitch = (geom[11] - 1) * geom[9] + geom[5];
+  const int64_t plane = rows * pitch, budget = DC_SMEM_BYTES / 4;
+  int64_t cc = 0;
+  if (stage_input && plane < budget) {
+    cc = budget / (plane + static_cast<int64_t>(p->khw) * (DC_CG + 1) + 4);
+    if (cc > p->C) cc = p->C;
+    while (cc > 0 && (cc * plane + 3) / 4 * 4 + cc * p->khw * (DC_CG + 1) > budget) --cc;
+  }
+  if (cc == 0) {   // weights + (ci, kr, kc) of each tap of a 512-tap chunk: (8 + 3) * 512 * 4 bytes = 22 KB
+    p->cc = 0; p->rows = p->pitch = p->plane = 0;
+    p->ws_off = 0;
+    p->toff_off = DC_KC * DC_CG;
+    return false;
+  }
+  p->cc = static_cast<int>(cc);
+  p->rows = static_cast<int>(rows); p->pitch = static_cast<int>(pitch); p->plane = static_cast<int>(plane);
+  p->ws_off = static_cast<int>((cc * plane + 3) / 4 * 4);   // 16-byte aligned weights
+  p->toff_off = p->ws_off + static_cast<int>(cc) * p->khw * DC_CG;
+  return true;
+}
+
+template <bool MULTI, bool STAGED>
+__global__ void __launch_bounds__(256)
+conv2d_direct_kernel(float *__restrict__ out, const float *__restrict__ in, const float *__restrict__ ker, DirectConvParams p) {
+  __shared__ float4 dc_smem4[DC_SMEM_BYTES / 16];
+  float *smem = reinterpret_cast<float *>(dc_smem4);
+  float *ws = smem + p.ws_off;                                   // [tap][DC_CG] weights of the current chunk
+  int *toff = reinterpret_cast<int *>(smem + p.toff_off);        // STAGED: tap -> window offset; else (ci, kr, kc) x 512
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  if constexpr (STAGED) {   // the same for every chunk: channel-local tap tl -> (tl / khw) * plane + kr * pitch + kc
+    for (int tl = tid; tl < p.cc * p.khw; tl += 256) {
+      const int ci = tl / p.khw, r = tl - ci * p.khw, kr = r / p.kW;
+      toff[tl] = ci * p.plane + kr * p.pitch + (r - kr * p.kW);
+    }
+  }
+  for (int64_t t = blockIdx.x; t < p.total; t += gridDim.x) {
+    const int g = static_cast<int>(t % p.groups);
+    const int64_t rest = t / p.groups;
+    const int tile = static_cast<int>(rest % p.tiles);
+    const int64_t n = rest / p.tiles;
+    const int co0 = g * DC_CG, p0 = tile * DC_PIX, oh_a = p0 / p.outW;
+    const float *img = in + n * static_cast<int64_t>(p.C) * p.H * p.W;
+    const int64_t HW = static_cast<int64_t>(p.H) * p.W;
+    int base[DC_CPT], ih0[DC_CPT], iw0[DC_CPT];   // STAGED: window offset of the pixel's first tap; else its image position
+    bool live[DC_CPT];
+#pragma unroll
+    for (int j = 0; j < DC_CPT; ++j) {
+      const int pix = p0 + tid + j * 256;
+      live[j] = pix < p.outHW;
+      const int oh = live[j] ? pix / p.outW : oh_a, ow = live[j] ? pix - oh * p.outW : 0;
+      base[j] = (oh - oh_a) * p.sH * p.pitch + ow * p.sW;
+      ih0[j] = oh * p.sH - p.pH;
+      iw0[j] = ow * p.sW - p.pW;
+    }
+    float acc[DC_CPT][DC_CG], x[DC_CPT][DC_CG];
+#pragma unroll
+    for (int j = 0; j < DC_CPT; ++j)
+#pragma unroll
+      for (int c = 0; c < DC_CG; ++c) { acc[j][c] = 0.0f; x[j][c] = 0.0f; }
+    // end of a summation block: x = x + blk (x starts at +0: the exact GEMM's beta = 0 epilogue, then beta' = 1)
+    auto flush = [&]() {
+#pragma unroll
+      for (int j = 0; j < DC_CPT; ++j)
+#pragma unroll
+        for (int c = 0; c < DC_CG; ++c) { x[j][c] = __fadd_rn(x[j][c], acc[j][c]); acc[j][c] = 0.0f; }
+    };
+    auto fma_tap = [&](const float *w, const float *v) {
+#pragma unroll
+      for (int j = 0; j < DC_CPT; ++j)
+#pragma unroll
+        for (int c = 0; c < DC_CG; ++c) acc[j][c] = __fmaf_rn(w[c], v[j], acc[j][c]);
+    };
+    if constexpr (STAGED) {
+      const int ih_a = oh_a * p.sH - p.pH;
+      for (int c0 = 0; c0 < p.C; c0 += p.cc) {
+        const int cn = p.C - c0 < p.cc ? p.C - c0 : p.cc;
+        __syncthreads();   // the previous chunk (or tile) is consumed
+        // input: one warp per staged row, lanes along it (window column q <-> image column q - pW)
+        for (int rr = warp; rr < cn * p.rows; rr += 8) {
+          const int ci = rr / p.rows, ih = ih_a + (rr - ci * p.rows);
+          float *dst = smem + static_cast<int64_t>(rr) * p.pitch;
+          if (static_cast<unsigned>(ih) < static_cast<unsigned>(p.H)) {
+            const float *src = img + (c0 + ci) * HW + static_cast<int64_t>(ih) * p.W;
+            for (int q = lane; q < p.pitch; q += 32) {
+              const int iw = q - p.pW;
+              dst[q] = static_cast<unsigned>(iw) < static_cast<unsigned>(p.W) ? src[iw] : 0.0f;
+            }
+          } else {
+            for (int q = lane; q < p.pitch; q += 32) dst[q] = 0.0f;
+          }
+        }
+        for (int i = tid; i < cn * p.khw * DC_CG; i += 256) {
+          const int tl = i / DC_CG, c = i - tl * DC_CG;
+          ws[i] = co0 + c < p.Cout ? ker[static_cast<int64_t>(co0 + c) * p.K + c0 * p.khw + tl] : 0.0f;
+        }
+        __syncthreads();
+        const int taps = cn * p.khw, kk0 = c0 * p.khw;
+#pragma unroll 2
+        for (int tl = 0; tl < taps; ++tl) {
+          const float4 wa = reinterpret_cast<const float4 *>(ws)[2 * tl], wb = reinterpret_cast<const float4 *>(ws)[2 * tl + 1];
+          const float w[DC_CG] = {wa.x, wa.y, wa.z, wa.w, wb.x, wb.y, wb.z, wb.w};
+          const int off = toff[tl];
+          float v[DC_CPT];
+#pragma unroll
+          for (int j = 0; j < DC_CPT; ++j) v[j] = smem[base[j] + off];
+          fma_tap(w, v);
+          if constexpr (MULTI) {
+            if (((kk0 + tl + 1) & (DC_KC - 1)) == 0) flush();   // block boundaries follow kk, not the channel chunks
+          }
+        }
+      }
+      if constexpr (MULTI) {
+        if (p.K & (DC_KC - 1)) flush();   // the last, partial block
+      }
+    } else {
+      int *tci = toff, *tkr = toff + DC_KC, *tkc = toff + 2 * DC_KC;
+      for (int k0 = 0; k0 < p.K; k0 += DC_KC) {   // one chunk = one summation block
+        const int kn = p.K - k0 < DC_KC ? p.K - k0 : DC_KC;
+        __syncthreads();
+        for (int i = tid; i < kn * DC_CG; i += 256) {
+          const int tl = i / DC_CG, c = i - tl * DC_CG;
+          ws[i] = co0 + c < p.Cout ? ker[static_cast<int64_t>(co0 + c) * p.K + k0 + tl] : 0.0f;
+        }
+        for (int tl = tid; tl < kn; tl += 256) {
+          const int kk = k0 + tl, ci = kk / p.khw, r = kk - ci * p.khw, kr = r / p.kW;
+          tci[tl] = ci; tkr[tl] = kr; tkc[tl] = r - kr * p.kW;
+        }
+        __syncthreads();
+        for (int tl = 0; tl < kn; ++tl) {
+          const float *w = ws + tl * DC_CG;
+          const int kr = tkr[tl], kc = tkc[tl];
+          const float *plane = img + tci[tl] * HW;
+          float v[DC_CPT];
+#pragma unroll
+          for (int j = 0; j < DC_CPT; ++j) {
+            const int ih = ih0[j] + kr, iw = iw0[j] + kc;
+            v[j] = live[j] && static_cast<unsigned>(ih) < static_cast<unsigned>(p.H) &&
+                           static_cast<unsigned>(iw) < static_cast<unsigned>(p.W)
+                       ? plane[static_cast<int64_t>(ih) * p.W + iw]
+                       : 0.0f;
+          }
+          float wr[DC_CG];
+#pragma unroll
+          for (int c = 0; c < DC_CG; ++c) wr[c] = w[c];
+          fma_tap(wr, v);
+        }
+        if constexpr (MULTI) flush();
+      }
+    }
+    // the single store: act(x + bias[co]) for every live pixel of the group's channels
+    const bool has_epi = p.bias != nullptr || p.act != 0;
+#pragma unroll
+    for (int c = 0; c < DC_CG; ++c) {
+      if (co0 + c >= p.Cout) break;
+      float *oplane = out + (n * p.Cout + co0 + c) * static_cast<int64_t>(p.outHW);
+#pragma unroll
+      for (int j = 0; j < DC_CPT; ++j) {
+        if (!live[j]) continue;
+        float v = MULTI ? x[j][c] : __fadd_rn(0.0f, acc[j][c]);
+        if (has_epi) v = simt_bias_act(v, p.bias, 1, p.act, co0 + c, p0 + tid + j * 256);
+        oplane[p0 + tid + j * 256] = v;
+      }
     }
   }
 }

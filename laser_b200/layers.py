@@ -7,6 +7,7 @@
     conv2d_out_shape, im2col_workspace_size       benchmarks/convolution/conv2d_common.nim:15-45,
                                                   conv2d_im2col.nim:8-18
     im2col, conv2d_im2col                         conv2d_im2col.nim:44-166
+    conv2d_direct                                 conv2d_direct_convolution.nim:8-76
     gemm_strided_batched                          (roadmap item of the reference, README.md:253-263)
     copyFrom(dst, src)                            laser/tensor/initialization.nim:80-112
 
@@ -17,14 +18,14 @@ import ctypes
 
 import numpy as np
 
-from ._capi import PATH_AUTO, check, lib
+from ._capi import PATH_AUTO, Epilogue, check, lib
 from .gemm import _current_stream, _resolve, _scalar
 from .tensor import _ITEMSIZE, Tensor
 
 FOREACH_OPS = {"copy": 0, "fill": 1, "scale": 2, "add": 3, "sub": 4, "mul": 5, "fma": 6, "axpy": 7, "bench": 8}
 
 __all__ = ["forEach", "FOREACH_OPS", "transpose2D_copy", "transpose2D_batched", "nchw2nhwc", "nhwc2nchw", "conv2d_out_shape",
-           "im2col_workspace_size", "im2col", "conv2d_im2col", "gemm_strided_batched", "copyFrom"]
+           "im2col_workspace_size", "im2col", "conv2d_im2col", "conv2d_direct", "gemm_strided_batched", "copyFrom"]
 
 _i64 = ctypes.c_int64
 
@@ -126,6 +127,38 @@ def conv2d_im2col(output, input, ishape, kernel, kshape, padding, strides, works
     pw = _dev_f32(workspace) if workspace is not None else 0
     check(lib().laser_b200_conv2d_im2col_f32_dev(po, pi, _i4(ishape), pk, _i4(kshape), _i2(padding), _i2(strides), pw,
                                                  int(workspace_images), int(path), stream))
+
+
+ACTIVATIONS = {"none": 0, "relu": 1, "tanh": 2, "sigmoid": 3}
+
+
+def conv2d_direct(output, input, ishape, kernel, kshape, padding, strides, bias=None, activation=None, stream=None):
+    """NCHW convolution without a workspace, one kernel launch per call; bit for bit what conv2d_im2col returns on
+    path=PATH_SIMT.  numpy arrays: host entry (synchronous, no epilogue: `bias` / `activation` are a TypeError);
+    device pointers: `bias` (NULL or a float32 device vector of c_out values) and `activation` (none | relu | tanh |
+    sigmoid, or its code) are applied once to the final sum, act(x + bias[c_out])."""
+    po, to, do = _resolve(output)
+    pi, ti, di = _resolve(input)
+    pk, tk, dk = _resolve(kernel)
+    if not (to == ti == tk == "f32"):
+        raise TypeError("conv2d_direct is float32 only")
+    if not (do == di == dk):
+        raise TypeError("output, input, kernel must all be host pointers or all be device pointers")
+    if not do:
+        if bias is not None or activation is not None:
+            raise TypeError("the host-pointer entry has no epilogue: bias and activation need device buffers")
+        check(lib().laser_b200_conv2d_direct_f32(po, pi, _i4(ishape), pk, _i4(kshape), _i2(padding), _i2(strides)))
+        return
+    epi = None
+    if bias is not None or activation is not None:
+        epi = Epilogue()
+        if bias is not None:
+            epi.bias = _dev_f32(bias)
+        epi.bias_per_row = 1
+        epi.activation = ACTIVATIONS[activation] if isinstance(activation, str) else int(activation or 0)
+    stream = _current_stream() if stream is None else stream
+    check(lib().laser_b200_conv2d_direct_f32_dev(po, pi, _i4(ishape), pk, _i4(kshape), _i2(padding), _i2(strides),
+                                                 ctypes.byref(epi) if epi is not None else None, stream))
 
 
 def gemm_strided_batched(batch, M, N, K, alpha, A, rowStrideA, colStrideA, batchStrideA, B, rowStrideB, colStrideB,

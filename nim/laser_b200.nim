@@ -241,6 +241,11 @@ proc laser_b200_conv2d_out_shape*(ishape, kshape: ptr array[4, int64], padding, 
                                   oshape: ptr array[4, int64]): cint
 proc laser_b200_conv2d_im2col_f32*(output, input: ptr float32, ishape: ptr array[4, int64], kernel: ptr float32,
                                    kshape: ptr array[4, int64], padding, strides: ptr array[2, int64]): cint
+proc laser_b200_conv2d_direct_f32*(output, input: ptr float32, ishape: ptr array[4, int64], kernel: ptr float32,
+                                   kshape: ptr array[4, int64], padding, strides: ptr array[2, int64]): cint
+proc laser_b200_conv2d_direct_f32_dev*(output, input: ptr float32, ishape: ptr array[4, int64], kernel: ptr float32,
+                                       kshape: ptr array[4, int64], padding, strides: ptr array[2, int64],
+                                       epi: pointer, stream: pointer): cint
 {.pop.}
 
 proc transpose2D_copy*[T](dst, src: ptr (T or UncheckedArray[T]), NR, NC: Natural) =
@@ -269,3 +274,14 @@ proc conv2d_im2col*(output: ptr float32, oshape: TensorShape, input: ptr float32
     pad = [padding.h.int64, padding.w.int64]
     st = [strides.h.int64, strides.w.int64]
   check laser_b200_conv2d_im2col_f32(output, input, ish.addr, kernel, ksh.addr, pad.addr, st.addr)
+
+proc conv2d_direct*(output: ptr float32, oshape: TensorShape, input: ptr float32, ishape: TensorShape,
+                    kernel: ptr float32, kshape: KernelShape, padding: Padding, strides: Strides) =
+  ## conv2d_direct_convolution.nim:8-76 (host pointers, synchronous): no workspace, one kernel launch; `output` is
+  ## overwritten (the reference adds into a zeroed one) with the values conv2d_im2col gives on the exact path
+  var
+    ish = [ishape.n.int64, ishape.c.int64, ishape.h.int64, ishape.w.int64]
+    ksh = [kshape.c_out.int64, kshape.c_in.int64, kshape.kH.int64, kshape.kW.int64]
+    pad = [padding.h.int64, padding.w.int64]
+    st = [strides.h.int64, strides.w.int64]
+  check laser_b200_conv2d_direct_f32(output, input, ish.addr, kernel, ksh.addr, pad.addr, st.addr)
